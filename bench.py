@@ -199,8 +199,9 @@ def c5_cpu(wl, data_host, qh, n_queries, threads):
     return n_queries / (time.perf_counter() - t0), res
 
 
-def c5_measure(ctx, torch, dev, wl, steps, warmup, cpu_sample=True):
-    """BASELINE configs[4] on one context: returns the record (value, breakdown, tensor roofline, e2e, cpu sample)."""
+def c5_measure(ctx, torch, dev, wl, steps, warmup, cpu_sample=True, dump_dir=None):
+    """BASELINE configs[4] on one context: returns the record (value, breakdown, tensor roofline, e2e, cpu sample).
+    With dump_dir, the results of the last timed call are written there."""
     import numpy as np
     n, d, nq, k, metric = wl["n"], wl["d"], wl["nq"], wl["k"], wl["metric"]
     cores = os.cpu_count() or 1
@@ -225,6 +226,8 @@ def c5_measure(ctx, torch, dev, wl, steps, warmup, cpu_sample=True):
     dev_ms = ctx.timer_stop()
     wall = time.perf_counter() - t0
     c1 = ctx.counters()
+    if dump_dir:
+        write_outputs(dump_dir, rerank_outputs(out))
     bd = {kk: sum(b[kk] for b in gemm_ms) / len(gemm_ms) for kk in gemm_ms[0]}
     stats = ctx.rerank_stats()
     peak, peak_src = tensor_peak(burst=True)
@@ -302,7 +305,8 @@ def run_c5(args, wl):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    rec = c5_measure(ctx, torch, dev, wl, args.steps, args.warmup, cpu_sample=(rank == 0 and not args.no_cpu_baseline))
+    rec = c5_measure(ctx, torch, dev, wl, args.steps, args.warmup, cpu_sample=(rank == 0 and not args.no_cpu_baseline),
+                     dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
     t_ms = torch.tensor([rec["ms_per_step"]], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -426,6 +430,7 @@ def timed_builds(rig, wl, items, seeds, steps, warmup):
 
     for _ in range(warmup):
         one_step()
+    counts = None
     c0 = ctx.counters()
     sampler = ClockSampler(rig.local_rank)
     rig.barrier()
@@ -437,7 +442,7 @@ def timed_builds(rig, wl, items, seeds, steps, warmup):
     alg_bytes = 0
     shadow_acc = {}
     for _ in range(steps):
-        one_step()
+        counts = one_step()
         sr = ctx.build_stats()["scanned_rows"]
         sh = ctx.build_shadow_stats()
         scanned += sr
@@ -455,7 +460,8 @@ def timed_builds(rig, wl, items, seeds, steps, warmup):
     st, bd = ctx.build_stats(), ctx.build_breakdown()
     return {"alg_bytes_per_step": ab_step, "shadow_rows_per_step": {k: v / steps for k, v in shadow_acc.items()}, "last_step_alg_bytes": scan_bytes(st["scanned_rows"], ctx.build_shadow_stats(), d),
             "ms_per_step": ms_per_step, "value": n / (ms_per_step * 1e-3), "wall_ms_per_step": wall * 1e3 / steps, "clocks": clocks,
-            "launches": int(c1["launches"] - c0["launches"]), "scanned_rows_per_step": sc, "stats": st, "breakdown": bd, "my_trees": my_trees}
+            "launches": int(c1["launches"] - c0["launches"]), "scanned_rows_per_step": sc, "stats": st, "breakdown": bd, "my_trees": my_trees,
+            "last_step_counts": counts}
 
 
 def build_record(wl, tb, world):
@@ -469,6 +475,116 @@ def build_record(wl, tb, world):
             "scan_rows_per_step": tb["shadow_rows_per_step"],
             "schedule": "lockstep" if os.environ.get("ARROY_B200_LOCKSTEP") else ("persistent: one cooperative launch per wave (control CTA per tree + worker CTAs)" if tb["stats"]["steps"] == 1 else "async per-tree graph branches (control / work kernel per attempt)"),
             "misspeculated_two_means": tb["stats"].get("misspeculated_splits", 0.0), "breakdown_ms_last_step": tb["breakdown"]}
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed in its last step, so that two builds of the project can be compared
+# output for output (the inputs are the same seeded stream in every run)
+# ---------------------------------------------------------------------------------------------------------------------
+
+DUMP_LIMIT_BYTES = 64 << 20
+# seeded samples keep the dump of c4 (100 trees over 10M x 1536) under the limit; c2 fits whole but for the normals (~300 MB)
+DUMP_NODES, DUMP_SPLIT_NORMALS, DUMP_ITEMS = 1 << 18, 4096, 16384
+
+
+def write_outputs(out_dir, arrays):
+    """{name: array} -> out_dir/<name>.npy; float32 arrays stay float32, all others become float64 (u32 ids are exact there)."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError("outputs to dump take %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def roaring_ids(b, o):
+    """Item ids of the RoaringBitmap serialized at b[o:] (portable format without run containers, as NodeCodec writes it)."""
+    import numpy as np
+    cookie, n = np.frombuffer(b, dtype="<u4", count=2, offset=o)
+    if cookie != 12346:
+        raise ValueError("unexpected roaring cookie %d" % cookie)
+    keys = np.frombuffer(b, dtype="<u2", count=2 * int(n), offset=o + 8).reshape(-1, 2)
+    offs = np.frombuffer(b, dtype="<u4", count=int(n), offset=o + 8 + 4 * int(n))
+    parts = []
+    for (key, card_m1), off in zip(keys.tolist(), offs.tolist()):
+        if card_m1 + 1 > 4096:   # bitmap container
+            low = np.flatnonzero(np.unpackbits(np.frombuffer(b, dtype=np.uint8, count=8192, offset=o + off), bitorder="little"))
+        else:                    # array container
+            low = np.frombuffer(b, dtype="<u2", count=card_m1 + 1, offset=o + off)
+        parts.append((key << 16) | low.astype(np.int64))
+    return np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
+
+
+def forest_outputs(ctx, wl, counts):
+    """The forest that the last build_trees_begin left parked on the device, emitted as a caller receives it (node ids numbered
+    like a one-GPU Writer::build: roots 0..T-1, then tree by tree, last tree first) and laid out as arrays:
+      node_counts            [T]              nodes per tree, root included (what build_trees_begin returns)
+      split_nodes            [<=2^18, 3 + h]  node id, left child, right child, header of the normal (NaN: no normal)
+      split_normal_ids       [<=4096]         seeded sample of the split nodes ...
+      split_normals          [<=4096, d]      ... and their normals (f32; NaN: no normal)
+      descendants            [<=2^18, 2]      node id, number of items of the Descendants nodes
+      sampled_items          [<=16384]        seeded sample of the item ids ...
+      leaf_of_sampled_items  [T, <=16384]     ... and the Descendants node holding each of them in every tree
+    Tables with more rows than shown are a seeded sample of their rows, in node id order."""
+    import struct
+
+    import numpy as np
+    import arroy_b200 as ab
+    from arroy_b200 import parallel
+    n, d, T, metric = wl["n"], wl["d"], wl["n_trees"], wl["metric"]
+    counts = np.asarray(counts, dtype=np.int64)
+    base = parallel.node_id_bases(counts, T)
+    arena = ab.Arena()
+    ctx.build_trees_emit(list(range(T)), base, arena=arena)
+    n_ids = T + int((counts - 1).sum())
+    tree_of = np.empty(n_ids, dtype=np.int64)
+    tree_of[:T] = np.arange(T)
+    for t in range(T):
+        tree_of[int(base[t]):int(base[t]) + int(counts[t]) - 1] = t
+    hf = 2 if metric == "dot-product" else 1
+
+    def sample(n_rows, k, seed):
+        return np.sort(np.random.default_rng(seed).choice(n_rows, min(n_rows, k), replace=False))
+    items = sample(n, DUMP_ITEMS, 0)
+    slot = np.full(n, -1, dtype=np.int64)   # item ids are the rows 0..n-1 here
+    slot[items] = np.arange(len(items))
+    leaf = np.full((T, len(items)), -1.0)
+    splits, desc = [], []
+    for nid in range(n_ids):
+        b = arena.get(nid)
+        if b is None:
+            raise RuntimeError("node %d was not emitted" % nid)
+        if b[0] == 1:
+            ids = roaring_ids(b, 1)
+            desc.append((nid, len(ids)))
+            s = slot[ids]
+            leaf[tree_of[nid], s[s >= 0]] = nid
+        else:
+            left, right = struct.unpack_from(">II", b, 1)
+            hdr = np.frombuffer(b, dtype=np.float32, count=hf, offset=9).tolist() if len(b) > 9 else [float("nan")] * hf
+            splits.append([nid, left, right] + hdr)
+    splits = np.array(splits, dtype=np.float64).reshape(-1, 3 + hf)
+    desc = np.array(desc, dtype=np.float64).reshape(-1, 2)
+    normal_ids = splits[sample(len(splits), DUMP_SPLIT_NORMALS, 1), 0]
+    normals = np.full((len(normal_ids), d), np.nan, dtype=np.float32)
+    for r, nid in enumerate(normal_ids):
+        b = arena.get(int(nid))
+        if len(b) > 9:
+            normals[r] = np.frombuffer(b, dtype=np.float32, count=d, offset=9 + 4 * hf)
+    del arena
+    return {"node_counts": counts, "split_nodes": splits[sample(len(splits), DUMP_NODES, 2)], "split_normal_ids": normal_ids,
+            "split_normals": normals, "descendants": desc[sample(len(desc), DUMP_NODES, 3)], "sampled_items": items, "leaf_of_sampled_items": leaf}
+
+
+def rerank_outputs(out):
+    """rerank_shared results: ids and distances per query (NaN past the query's result length)."""
+    import numpy as np
+    rows, dist, length = out
+    valid = np.arange(rows.shape[1])[None, :] < length[:, None]
+    return {"rerank_ids": np.where(valid, rows.astype(np.float64), np.nan), "rerank_distances": np.where(valid, dist, np.float32(np.nan)),
+            "rerank_lengths": length}
 
 
 def leaf_blob(rig, wl, items):
@@ -714,7 +830,16 @@ def main():
     ap.add_argument("--no-headline", action="store_true", help="skip the 10M x 768 sub-record of the default workload")
     ap.add_argument("--no-c5", action="store_true", help="skip the config-5 sub-record of the default workload")
     ap.add_argument("--queries", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (f32 / f64, at most 64 MB; "
+                         "seeded samples of larger outputs), for comparing two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
+    if args.dump_outputs and args.workload != "c5" and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs of a forest build needs one process (each rank holds only its own trees)")
     wl = WORKLOADS[args.workload]
     if args.workload == "c5":
         run_c5(args, wl)
@@ -733,6 +858,8 @@ def main():
     items = synth_items(rig, wl)     # generated on the device of rank 0 (counter-based ChaCha12 stream)
     seeds = derive_seeds(rig.ab, T)
     tb = timed_builds(rig, wl, items, seeds, args.steps, args.warmup)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, forest_outputs(ctx, wl, tb["last_step_counts"]))
     line = {
         "metric": "index-build vectors/sec", "value": tb["value"], "unit": "vectors/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": tb["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",

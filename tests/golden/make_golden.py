@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Regenerate tests/golden/*.json from the reference's own test expectations.
 
-Run in the authoring container only (needs /root/reference, which does not exist on the
-GPU box): `python tests/golden/make_golden.py`. It parses the *expected values* held by
+Needs a checkout of the reference crate (arroy) and is not part of the test run:
+`python tests/golden/make_golden.py <path of the arroy checkout>`. It parses the *expected values* held by
 the reference's tests — the insta `.snap` files under src/tests/snapshots/ and the inline
 snapshots in src/tests/writer.rs / src/tests/reader.rs / src/tests/upgrade.rs — into small
 JSON fixtures. No reference source code is copied; only golden numbers (node ids, child
@@ -13,7 +13,7 @@ import os
 import re
 import sys
 
-REF = "/root/reference"
+REF = None   # the reference checkout, from the command line
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 TREE_SPLIT = re.compile(
@@ -96,8 +96,10 @@ def inline_snapshots(path):
 
 
 def main():
-    if not os.path.isdir(REF):
-        sys.exit("needs /root/reference")
+    global REF
+    if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "src", "tests")):
+        sys.exit("usage: make_golden.py <path of the arroy checkout>")
+    REF = sys.argv[1]
     g = {}
     g["lot_of_random_points"] = snap_file("arroy__tests__writer__write_and_update_lot_of_random_points.snap")
     # second snapshot of the same test: only its *items* are used (even ids redrawn after the

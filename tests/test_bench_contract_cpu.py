@@ -29,5 +29,11 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert "workload" in j["config"]
 
 
+def test_bad_step_counts_and_dump_of_the_reference_arm_are_refused():
+    for args in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c1"] + args, capture_output=True, text=True, timeout=60, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, args
+
+
 def test_reference_arm_only_runs_on_rank_zero():
     assert _run(["--impl", "reference", "--workload", "c1", "--steps", "1", "--warmup", "1"], env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}) == []
